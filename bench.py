@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            (N>1: launched by torchrun, one rank per GPU)
   python bench.py --impl reference --gpus N --steps K --warmup W   (the reference's CPU path, restated; rank 0 only)
+  python bench.py ... --dump-outputs DIR   (also writes the last timed step's next_ids / logits: dump_outputs())
 
 A "step" is one decode step of the full 28-layer stack + lm_head + greedy sampling for a batch of B sequences at
 context ctx, replayed from a CUDA graph.  Prints ONE JSON line (see DESIGN.md "Measurement"):
@@ -242,13 +243,36 @@ def step_roofline(st, ctx, ms_per_step, hbm_peak):
             "roofline_tok_s": round(st.B / (sb / (hbm_peak * 1e9)), 1)}
 
 
+DUMP_BYTES = 64_000_000
+
+
+def dump_outputs(st, out_dir):
+    """What the last timed step handed its caller, as DIR/<name>.npy: next_ids (the sampled token ids, float64) and logits
+    (float32 [batch, vocab]; under --tp N rank 0's vocabulary shard).  Logits beyond DUMP_BYTES in all are cut to a fixed
+    seeded sample of vocabulary columns, whose indices go to logits_columns (float64)."""
+    import numpy as np
+    ids = st.next_ids.cpu().numpy().astype(np.float64)
+    logits = st.logits.float().cpu().numpy()
+    out = {"next_ids": ids}
+    B, V = logits.shape
+    if ids.nbytes + logits.nbytes > DUMP_BYTES:
+        n = (DUMP_BYTES - ids.nbytes) // (4 * B + 8)
+        cols = np.sort(np.random.default_rng(0).choice(V, n, replace=False))
+        out["logits_columns"] = cols.astype(np.float64)
+        logits = logits[:, cols]
+    out["logits"] = logits
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def measure_tp(args, world, rank, hbm_peak, torch, dist):
     """Config C4 (BASELINE.json): ONE Qwen2-72B IQ-int4 instance, tensor parallel over all ranks of the job (QKV / gate / up
     column split, o / down row split + all-reduce, vocab-split lm_head), batch 16, ctx 4096, bf16 KV."""
     from b200spark import model
     cfg = model.QWEN2_72B
     B, ctx = args.tp_batch, args.tp_ctx
-    K, W = max(5, min(args.steps, 20)), 3
+    K, W = args.steps, 3
     t0 = time.time()
     st = model.DecodeStack(cfg, B, ctx + 3 * K + W + 16, wbits=4, group=-1, kv="none", span=128, tp_rank=rank, tp_size=world,
                            layers=args.tp_layers)
@@ -296,6 +320,8 @@ def run_gpu(args):
     ids = torch.randint(0, cfg.vocab, (B,), generator=torch.Generator().manual_seed(4321), dtype=torch.int64)
     st.ids.copy_(ids.cuda())
     ms, clocks = timed_steps(st, K, W, torch, dist, world, ClockSampler(local) if rank == 0 else None)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(st, args.dump_outputs)
     replicas = 1 if tp > 1 else world  # TP: the ranks share one batch; replicas: every rank has its own
     value = replicas * B * K / (ms * 1e-3)
     e2e_s = e2e_steps(st, ids, K, torch, dist, world)
@@ -446,7 +472,13 @@ def main():
     ap.add_argument("--tp-batch", type=int, default=16)
     ap.add_argument("--tp-ctx", type=int, default=4096)
     ap.add_argument("--tp-layers", type=int, default=None, help="debug: fewer layers in the TP record (INVALID as a bench number)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the next_ids / logits of the last timed step as DIR/<name>.npy (float32 / float64, <= 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the b200spark arm's outputs")
     if args.impl == "reference":
         run_reference(args)
     else:

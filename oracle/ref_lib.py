@@ -1,7 +1,7 @@
 """ctypes door to oracle/_ref/libdashinfer_ref.so — the UNMODIFIED reference GPU code (span-attention library + the
-span-cache writers) built by oracle/build_ref.py.  TEST INFRASTRUCTURE: only tests/ import this.
+span-cache writers) built by oracle/build_ref.py.  TEST INFRASTRUCTURE: only tests/golden/make_ref_pin.py imports this.
 
-    load() -> lib or None          (None when the library was never built: tests skip with the reason)
+    load() -> lib or None          (None when the library was never built)
     span_attn(lib, out, q, k_tab, v_tab, lens_host, nH, nG, span, n_spans, qmode, scale)
     cache_append(lib, k_tab, v_tab, q_out, qkv, old_lens_u32, nH, nG, span, n_spans, qmode)
     context_span_copy(lib, span_ptrs, src, nG, span, seq_len, qmode)

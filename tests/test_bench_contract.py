@@ -1,9 +1,11 @@
 """CPU: the bench.py JSON-line contract on the arm that runs without a GPU (`--impl reference`, tiny config), and that the
-product arm refuses to run without a GPU instead of falling back."""
+product arm refuses to run without a GPU instead of falling back.  GPU: the outputs --dump-outputs writes."""
 import json
 import os
 import subprocess
 import sys
+
+import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -64,3 +66,50 @@ def test_reference_arm_sets_threads_under_torchrun():
     sys.path.insert(0, ROOT)
     import bench
     assert d["cpu_baseline"]["cores"] == bench.physical_cores()
+
+
+def test_steps_below_one_are_refused():
+    r = _run("--impl", "reference", "--model", "tiny", "--steps", "0")
+    assert r.returncode == 2 and "--steps" in r.stderr
+
+
+def test_dump_outputs_keeps_to_64_mb(tmp_path):
+    """Logits larger than the budget are cut to a seeded sample of vocabulary columns, the same from run to run."""
+    import numpy as np
+    import torch
+    from types import SimpleNamespace
+    sys.path.insert(0, ROOT)
+    import bench
+    logits = torch.randn(128, 152064, generator=torch.Generator().manual_seed(0)).to(torch.bfloat16)
+    st = SimpleNamespace(next_ids=logits.float().argmax(1), logits=logits)
+    for d in (tmp_path / "a", tmp_path / "b"):
+        bench.dump_outputs(st, str(d))
+    files = sorted(p.name for p in (tmp_path / "a").iterdir())
+    assert files == ["logits.npy", "logits_columns.npy", "next_ids.npy"]
+    assert sum(p.stat().st_size for p in (tmp_path / "a").iterdir()) <= 64_000_000
+    out = {f: np.load(tmp_path / "a" / f) for f in files}
+    cols = out["logits_columns.npy"]
+    assert cols.dtype == np.float64 and np.all(np.diff(cols) > 0) and cols[-1] < 152064
+    assert out["logits.npy"].dtype == np.float32
+    assert np.array_equal(out["logits.npy"], logits.float().numpy()[:, cols.astype(np.int64)])
+    assert np.array_equal(out["next_ids.npy"], st.next_ids.numpy())
+    for f in files:
+        assert np.array_equal(out[f], np.load(tmp_path / "b" / f))
+
+
+@pytest.mark.gpu
+def test_dump_outputs_of_the_last_timed_step(tmp_path):
+    """--dump-outputs writes the next_ids / logits of the last timed step; the same arguments give the same arrays."""
+    import numpy as np
+    dumps = []
+    for run in ("a", "b"):
+        d = tmp_path / run
+        r = _run("--model", "tiny", "--batch", "4", "--ctx", "64", "--steps", "3", "--warmup", "1", "--sub-batches", "",
+                 "--no-cpu", "--dump-outputs", str(d))
+        assert r.returncode == 0, r.stderr[-400:]
+        dumps.append({n: np.load(d / (n + ".npy")) for n in ("next_ids", "logits")})
+    ids, logits = dumps[0]["next_ids"], dumps[0]["logits"]
+    assert ids.dtype == np.float64 and logits.dtype == np.float32 and logits.shape == (4, 1024)
+    assert np.array_equal(ids, logits.argmax(1))
+    for n in ("next_ids", "logits"):
+        assert np.array_equal(dumps[0][n], dumps[1][n]), n
